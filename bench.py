@@ -2,11 +2,12 @@
 """Benchmark of the GeoFormer matching hot path (BASELINE.json metric: 640x480 pairs/s on B200;
 conf-matrix tensor-pipe fraction of peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the full forward (backbone -> coarse transformer -> coarse matching ->
 host RANSAC -> geo transformer -> coarse matching -> fine stage) over one batch of synthetic
-HPatches-shaped 640x480 pairs.  Prints ONE JSON line on rank 0.
+HPatches-shaped 640x480 pairs.  Prints ONE JSON line on rank 0.  Inputs and weights are seeded, so
+the outputs written by --dump-outputs can be compared between two builds of the project.
 """
 import argparse
 import copy
@@ -44,7 +45,13 @@ def parse():
     ap.add_argument("--hw", default=None, help="HxW override for informational runs of the other BASELINE configs (e.g. 768x768)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--stage-times", action="store_true", help="print a per-stage CUDA-event breakdown to stderr")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output arrays of the last timed step as DIR/<name>.npy "
+                         "(rank 0 only; float32, or float64 for float64 and integer outputs; at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def workload_config(args, extra=None):
@@ -57,6 +64,34 @@ def workload_config(args, extra=None):
     if extra:
         cfg.update(extra)
     return cfg
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(outputs, out_dir, limit=DUMP_LIMIT_BYTES):
+    """Write every tensor of one step's output dict as <out_dir>/<name>.npy: floating tensors as float32 (float64 stays
+    float64), integer and bool tensors as float64, which holds them exactly.  Above `limit` bytes in all, arrays of more
+    than one row keep a fixed, seeded sample of their rows (arrays of the same length keep the same rows), so that two
+    runs stay comparable row for row."""
+    arrs = {}
+    for k, v in outputs.items():
+        if not torch.is_tensor(v):
+            continue
+        a = v.detach().cpu().numpy()
+        arrs[k] = a.astype(np.float32 if np.issubdtype(a.dtype, np.floating) and a.dtype != np.float64 else np.float64)
+    big = [k for k, a in arrs.items() if a.ndim and a.shape[0] > 1]
+    rest = sum(a.nbytes for k, a in arrs.items() if k not in big)
+    total = rest + sum(arrs[k].nbytes for k in big)
+    if total > limit:
+        keep = (limit - rest) / (total - rest)
+        for k in big:
+            a = arrs[k]
+            rows = np.random.default_rng(0).choice(a.shape[0], max(1, int(a.shape[0] * keep)), replace=False)
+            arrs[k] = a[np.sort(rows)]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------- clocks
@@ -130,25 +165,25 @@ def cpu_forward_pairs_per_sec(steps, warmup, regime):
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
-    return 1.0 / float(np.mean(times)), torch.get_num_threads(), float(np.mean(times)), int(out["mkpts0_f"].shape[0])
+    return 1.0 / float(np.mean(times)), torch.get_num_threads(), float(np.mean(times)), out
 
 
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 4)), max(0, min(args.warmup, 1))
-    v, cores, spp, mf = cpu_forward_pairs_per_sec(steps, warmup, args.regime)
+    steps, warmup = args.steps, args.warmup
+    v, cores, spp, out = cpu_forward_pairs_per_sec(steps, warmup, args.regime)
+    if args.dump_outputs:
+        dump_outputs(out, args.dump_outputs)
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
             "warmup": warmup, "ms_per_step": 1e3 * spp, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic",
             "config": workload_config(args, {"pairs_per_step": 1,
-                                             "steps_note": f"CPU arm: each step is ONE pair (~2-5 s of all-core CPU work); requested "
-                                                           f"--steps {args.steps} / --warmup {args.warmup} clamped to {steps} / {warmup} "
-                                                           f"so that the run ends within a few minutes"}),
+                                             "steps_note": "CPU arm: each step is ONE pair (~2-5 s of all-core CPU work)"}),
             "cpu_baseline": {"value": v, "unit": UNIT, "cores": cores, "kind": "port",
                              "sample": f"{steps} single-pair {W}x{H} forwards of the CPU oracle port after {warmup} warm-up "
-                                       f"(the reference is pure PyTorch; /root/reference is absent on the GPU box)"},
+                                       f"(the reference is pure PyTorch; the oracle restates it op for op)"},
             "e2e": {"value": v, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     _emit(line)
 
@@ -198,13 +233,17 @@ def run_ours(args):
     xstream = torch.cuda.Stream(device=device)      # the path's only collective runs here, beside the next batches' compute
     xev = []                                        # CUDA events around every exchange (reported, not part of the timing)
     last_gather = {}
+    last_outputs = {}                               # --dump-outputs: the output tensors of the latest batch, in batch order
 
     def block_of(d):               # packed match list of the batch (device, fixed capacity, no host sync); pair id = global
         return pack_match_list(d["mkpts0_f"], d["mkpts1_f"], d["mconf"], d["m_bids"] * world + rank, cap)
 
     def counts_only(d):            # keep only what the report needs (frees the big per-batch tensors early)
         done_t.append(time.perf_counter())
-        return {"b_ids": d["b_ids"].shape[0], "mkpts0_f": d["mkpts0_f"].shape[0], "block": block_of(d)}
+        res = {"b_ids": d["b_ids"].shape[0], "mkpts0_f": d["mkpts0_f"].shape[0], "block": block_of(d)}
+        if args.dump_outputs:      # references only: no copy and no sync inside the timed loop
+            res["outputs"] = {k: v for k, v in d.items() if k not in ("image0", "image1")}
+        return res
 
     def to_host(d):                # what match_pairs() reads back (geoformer.py:53-54,73)
         k0, k1, cf = d["mkpts0_f"].cpu(), d["mkpts1_f"].cpu(), d["mconf"].cpu()
@@ -228,7 +267,9 @@ def run_ours(args):
         this: rank 0 issued extra all-gathers while the others waited in the final all-reduce)."""
         outs = []
         for res in pipe.run_iter(batches, post):
-            blk = (res[0] if isinstance(res, tuple) else res).pop("block")
+            r = res[0] if isinstance(res, tuple) else res
+            blk = r.pop("block")
+            last_outputs["outputs"] = r.pop("outputs", None)
             if collective:
                 exchange(blk)
             outs.append(res)
@@ -274,10 +315,13 @@ def run_ours(args):
     sampler.mark()
     done_t.clear()
     ms, outs, launches = timed(run_resident, args.steps)
+    step_outputs = last_outputs.pop("outputs", None)
     if os.environ.get("GF_BENCH_TRACE") and rank == 0:
         print("value loop, ms between batch completions:", " ".join(f"{1e3 * (b - a):.0f}" for a, b in zip(done_t, done_t[1:])),
               file=sys.stderr)
     ms_e2e, outs_e2e, _ = timed(run_e2e, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(step_outputs, args.dump_outputs)
     if rank == 0 and sampler.h is not None:      # same load once more, untimed, densely sampled (see ClockSampler)
         sampler.timed_samples = len(sampler.samples) - sampler.first
         sampler.interval = 0.04

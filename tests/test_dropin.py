@@ -2,11 +2,11 @@
 modules with ONE added line — ``sys.path.insert(0, "<repo>/geoformer_b200")`` (INTEGRATION.md §1).
 
 * CPU: a fresh interpreter with that line only executes the wrapper's three import statements
-  (eval_tool/immatch/modules/geoformer.py:6-10) and its ctor/load sequence (:23-31).  When /root/reference exists (the
-  build container) the UNMODIFIED wrapper class itself is constructed on top of the drop-in modules.
+  (eval_tool/immatch/modules/geoformer.py:6-10) and its ctor/load sequence (:23-31).  When GEOFORMER_REFERENCE names a
+  checkout of the reference repository, the UNMODIFIED wrapper class itself is constructed on top of the drop-in modules.
 * GPU: `match_inputs_` (:50-54,73) and `match_pairs` (:77-99) run through the top-level `model.*` imports on image
-  files; the matches are compared with the CPU oracle on the same resized tensors.  /root/reference does not exist on
-  the GPU box, so there the wrapper is the restatement below (same statements, same order).
+  files; the matches are compared with the CPU oracle on the same resized tensors.  Without a reference checkout the
+  wrapper is the restatement below (same statements, same order).
 """
 import os
 import subprocess
@@ -19,7 +19,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DROPIN = os.path.join(ROOT, "geoformer_b200")
-REFERENCE = "/root/reference"
+REFERENCE = os.environ.get("GEOFORMER_REFERENCE", "")      # optional checkout of the reference repository
 
 # what a maintainer adds on top of eval_Hpatches.py / eval_FIRE.py / eval_ISC.py / inference.py
 INTEGRATION_LINE = f"import sys; sys.path.insert(0, {DROPIN!r})"
@@ -84,9 +84,9 @@ def test_wrapper_imports_and_ctor_sequence_from_a_foreign_cwd(tmp_path):
     assert "DROPIN-OK" in _run(code, cwd=str(tmp_path))
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="/root/reference only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="needs GEOFORMER_REFERENCE: a checkout of the reference repository")
 def test_unmodified_reference_wrapper_constructs_on_the_dropin(tmp_path):
-    """The real `eval_tool.immatch.modules.geoformer.GeoFormer` (imported from /root/reference, unmodified) builds its
+    """The real `eval_tool.immatch.modules.geoformer.GeoFormer` (imported from the reference checkout, unmodified) builds its
     model from THIS repo's `model.*` and loads a checkpoint-shaped file through its own ctor."""
     ckpt = str(tmp_path / "geoformer.ckpt")
     _save_ckpt(ckpt)
@@ -170,7 +170,7 @@ WRAPPER_RESTATEMENT = textwrap.dedent("""
 def test_match_pairs_through_toplevel_model_imports(tmp_path):
     """Wrapper call sequence on image files, in a fresh interpreter that knows this repo only through the
     INTEGRATION.md line; result vs the CPU oracle on the same resized tensors (the unmodified reference wrapper is used
-    when /root/reference exists next to a GPU, the restatement above otherwise)."""
+    when a reference checkout is given, the restatement above otherwise)."""
     import cv2
     from geoformer_b200 import synth
     from oracle import geoformer_oracle as O

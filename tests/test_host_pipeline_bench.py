@@ -7,6 +7,7 @@ import subprocess
 import sys
 import time
 
+import numpy as np
 import pytest
 import torch
 
@@ -91,7 +92,7 @@ def test_bench_reference_arm_contract():
     assert r2.returncode == 0 and r2.stdout.strip() == ""
 
 
-def _dryrun(world, extra_env=None, timeout=420):
+def _dryrun(world, extra_env=None, timeout=420, extra_args=()):
     """bench.py's own arm on `world` simulated ranks (tests/bench_dryrun.py: operators emulated on CPU, gloo for NCCL)."""
     import socket
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
@@ -101,7 +102,8 @@ def _dryrun(world, extra_env=None, timeout=420):
                    MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), OMP_NUM_THREADS="2", GF_BENCH_EXTRA_HW="64x64,72x88",
                    **(extra_env or {}))
         procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "bench_dryrun.py"), "--gpus", str(world), "--steps", "3",
-                                       "--warmup", "1", "--batch", "2", "--hw", "64x96", "--no-cpu-baseline", "--depth", "2"],
+                                       "--warmup", "1", "--batch", "2", "--hw", "64x96", "--no-cpu-baseline", "--depth", "2",
+                                       *extra_args],
                                       stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, env=env, cwd=ROOT))
     outs = []
     deadline = time.time() + timeout
@@ -117,12 +119,14 @@ def _dryrun(world, extra_env=None, timeout=420):
 
 
 @pytest.mark.parametrize("world", [1, 2])
-def test_bench_own_arm_control_flow_dry_run(world):
+def test_bench_own_arm_control_flow_dry_run(world, tmp_path):
     """The whole of bench.py's own arm — warm-up, settle, both timed loops through MatchPipeline, the per-batch
     match-list exchange, barriers, max-over-ranks, the rank-0-only densely sampled pass, the diagnostics blocks and the
     JSON line — runs to completion on every simulated rank, rank 0 prints exactly one line with the contract's keys, the
-    other ranks print nothing.  (A collective issued by some ranks only would hang here as it would under NCCL.)"""
-    outs = _dryrun(world)
+    other ranks print nothing.  (A collective issued by some ranks only would hang here as it would under NCCL.)
+    --dump-outputs: rank 0 writes the output arrays of its last timed batch."""
+    dump = tmp_path / "outputs"
+    outs = _dryrun(world, extra_args=("--dump-outputs", str(dump)))
     assert outs is not None, "bench.py dry run timed out: the ranks' collective sequences differ"
     for rc, _, err in outs:
         assert rc == 0, err[-3000:]
@@ -144,6 +148,32 @@ def test_bench_own_arm_control_flow_dry_run(world):
     # the exchange gathered the last batch of EVERY rank
     per_rank = d["config"]["matches_fine_per_pair"] * 2
     assert d["config"]["gathered_matches_last_batch_all_ranks"] == pytest.approx(per_rank * world, rel=0.25)
+    got = {f.name[:-4]: np.load(f) for f in dump.iterdir()}
+    assert {"mkpts0_f", "mkpts1_f", "mconf", "m_bids", "b_ids", "i_ids", "j_ids"} <= set(got)
+    assert "image0" not in got and all(a.dtype in (np.float32, np.float64) for a in got.values())
+    n = got["mkpts0_f"].shape[0]
+    assert n > 0 and got["mkpts0_f"].shape == got["mkpts1_f"].shape == (n, 2) and got["mconf"].shape == got["m_bids"].shape == (n,)
+    assert set(np.unique(got["m_bids"])) <= {0.0, 1.0} and got["m_bids"].dtype == np.float64
+
+
+def test_bench_dump_outputs_dtypes_and_size_limit(tmp_path):
+    """bench.dump_outputs: floating tensors as float32 (float64 kept), integers as float64; above the byte limit every
+    multi-row array keeps a seeded sample of its rows (the same rows for arrays of the same length), small ones stay whole."""
+    code = (f"import sys, torch; sys.path.insert(0, {ROOT!r}); import bench\n"
+            "i = torch.arange(20000)\n"
+            "out = dict(x=torch.stack([i % 1000, i % 1000 + 1], 1).half(), i=i, d=i.double(), s=torch.tensor(7), t=(1, 2))\n"
+            f"bench.dump_outputs(out, {str(tmp_path / 'full')!r})\n"
+            f"bench.dump_outputs(out, {str(tmp_path / 'cut')!r}, limit=100000)\n")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=120, cwd=str(tmp_path))
+    assert r.returncode == 0, r.stderr[-2000:]
+    full = {k: np.load(tmp_path / "full" / f"{k}.npy") for k in ("x", "i", "d", "s")}
+    assert not (tmp_path / "full" / "t.npy").exists()
+    assert full["x"].dtype == np.float32 and full["i"].dtype == full["d"].dtype == full["s"].dtype == np.float64
+    assert np.array_equal(full["x"][:, 1] - 1, np.arange(20000) % 1000) and full["s"] == 7
+    cut = {k: np.load(tmp_path / "cut" / f"{k}.npy") for k in ("x", "i", "d", "s")}
+    assert sum(a.nbytes for a in cut.values()) <= 100000 and cut["s"] == 7
+    assert 0 < cut["i"].shape[0] < 20000 and np.all(np.diff(cut["i"]) > 0)
+    assert np.array_equal(cut["i"], cut["d"]) and np.array_equal(cut["x"][:, 0], cut["i"] % 1000)
 
 
 def test_bench_dry_run_detects_a_rank0_only_collective():
