@@ -61,6 +61,22 @@ def test_full_forward_gpu_tests_pass_on_emulated_operators(tmp_path):
     assert int(tail.split(" passed")[0].split()[-1]) >= 8, tail
 
 
+def test_emulations_pass_the_kernel_tests_at_scale(tmp_path):
+    """tests/test_gpu_kernels_at_scale.py with the operators emulated: its own host logic - the premise assertions (lazy
+    raises counted, leads in (6, 8], mixed warps, ring wraps, chunk sizes covered), the broken-reference sensitivity checks
+    and the fp64 references - runs in the CPU suite.  The batch-16 matcher case (several GB of fp32 confidences on the
+    CPU) is left to the GPU."""
+    dst = str(tmp_path / "emulated_test_gpu_kernels_at_scale.py")
+    emulated_copy(os.path.join(ROOT, "tests", "test_gpu_kernels_at_scale.py"), dst)
+    r = subprocess.run([sys.executable, "-m", "pytest", dst, "-q", "--no-header", "-p", "no:cacheprovider", "-p", "tests.conftest",
+                        "--rootdir", str(tmp_path), "-k", "not batch16"], capture_output=True, text=True, cwd=ROOT,
+                       timeout=1500)
+    tail = r.stdout.strip().splitlines()[-1] if r.stdout.strip() else r.stderr[-2000:]
+    assert r.returncode == 0, r.stdout[-6000:]
+    assert " passed" in tail and "failed" not in tail and "error" not in tail, tail
+    assert int(tail.split(" passed")[0].split()[-1]) >= 17, tail
+
+
 def test_smoke_entry_point_on_emulated_operators(monkeypatch, capsys):
     """__graft_entry__.smoke() (the driver's round-end check on cuda:0: shipped configuration vs the oracle) with the
     operators emulated: its own logic and thresholds hold when the arithmetic behind the contracts is exact."""
