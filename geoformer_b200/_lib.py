@@ -37,6 +37,11 @@ SIGNATURES = {
     "gf_linattn_reduce": (I, [P, I, P, I, I, I, I, I, P, P, P, P]),
     "gf_linattn_apply": (I, [P, I, P, P, P, I, I, I, I, I, P]),
     "gf_linattn_window": (I, [P, I, P, I, P, I, P, L, I, I, I, P]),
+    "gf_full_attention": (I, [P, I, P, I, P, I, P, I, I, I, I, I, P]),
+    "gf_dense_kv_h16": (I, [P, I, P, I, I, I, I, I, I, P, P, P, P]),
+    "gf_full_attention_tc": (I, [P, I, P, P, P, P, I, I, I, I, I, I, P]),
+    "gf_full_attention_window": (I, [P, I, P, I, P, I, P, L, I, I, I, P]),
+    "gf_full_attention_window_f16": (I, [P, I, P, I, P, I, P, L, I, I, I, P]),
     "gf_pack_split_f16": (I, [P, P, L, I, F, I, P]),
     "gf_similarity_f16x3": (I, [P, P, P, I, I, I, I, F, P]),
     "gf_similarity_ref": (I, [P, P, P, I, I, I, I, F, F, P]),

@@ -17,6 +17,10 @@
 //     the tensor core instead of 64 FADDs per row and tile);  out = O / l.
 // Operands are fp16 (kind::f16, fp32 accumulate).  The score matrix never touches HBM.
 // Roles: warp 0 TMA producer, warp 1 MMA issuer (+TMEM alloc), warps 2..5 softmax / epilogue.
+//
+// The same body runs LoFTR's full attention (loftr_module/linear_attention.py:54-85, `attention: 'full'`) at the coarse
+// level: heads x 32, dense keys (every query attends to all s tokens of its sample's source).  Per score the softmax work
+// is the same; the K tile shrinks to 64-byte rows (64B swizzle), the Q K^T MMA to two K = 16 steps and P V to N = 32.
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -29,19 +33,25 @@ extern std::atomic<int64_t> g_launches;
 namespace fa {
 constexpr int kBQ = 128;       // queries per CTA
 constexpr int kBK = 64;        // keys per tile
-constexpr int kD = 64;         // head dim
 constexpr int kRing = 4;       // K / V^T smem stages
-constexpr int kKBytes = kBK * 128;              // 64 keys x 64 dims (fp16): 8 KB
-constexpr int kVBytes = kD * 128;               // V^T tile: 64 dim rows x 64 keys (fp16): 8 KB
 constexpr int kOnesBytes = 16 * 128;            // B operand of the row-sum MMA: [16][64 keys] fp16, row 0 = 1
 constexpr int kSoftWarps = 4;
 constexpr int kThreads = 64 + 32 * kSoftWarps;
-constexpr int kRingBytes = kRing * (kKBytes + kVBytes);         // 64 KB; the epilogue stages the output here (32 KB)
-constexpr int kSmem = kRingBytes + kOnesBytes + 1024 + 256;
-constexpr int kTmemCols = 256;                  // S / P: 2 x 64 | O: 64 | l: 16 | Q: 32
-constexpr int kColO = 128, kColL = 192, kColQ = 208;
+constexpr int kTmemCols = 256;                  // S / P: 2 x 64 | O: D | l: 16 | Q: D / 2
 constexpr float kLazy = 8.f;                    // log2 units the reference maximum may lag behind
-static_assert(2 * kSmem <= 227 * 1024, "two CTAs per SM");
+// head dim 64 (geo self attention over anchors) or 32 (LoFTR coarse full attention over dense keys)
+template <int D>
+struct Cfg {
+  static_assert(D == 64 || D == 32, "head dim 64 or 32");
+  static constexpr int kKBytes = kBK * D * 2;   // 64 keys x D dims (fp16): 128 B rows (128B swizzle) or 64 B rows (64B)
+  static constexpr int kVBytes = D * 128;       // V^T tile: D dim rows x 64 keys (fp16)
+  static constexpr int kRingBytes = kRing * (kKBytes + kVBytes);   // the epilogue stages the output here (D x 512 B)
+  static constexpr int kSmem = kRingBytes + kOnesBytes + 1024 + 256;
+  static constexpr int kColO = 128, kColL = kColO + D, kColQ = kColL + 16;
+  static constexpr uint32_t kKDescHi = D == 64 ? ptx::kDescHiSw128 : ptx::kDescHiSw64;
+  static_assert(2 * kSmem <= 227 * 1024, "two CTAs per SM");
+  static_assert(kColQ + D / 2 <= kTmemCols, "tensor memory budget");
+};
 }  // namespace fa
 
 __device__ __forceinline__ float ex2_approx(float x) {
@@ -55,12 +65,17 @@ __device__ __forceinline__ uint32_t ex2_h2(float a, float b) {      // (2^a, 2^b
   return y;
 }
 
+// One CTA = (128-query tile, head, sample) over the first key_cnt[b] keys of the sample's K / V^T tiles (0: zeros).
+// D = 64: geo self attention over gathered anchors; D = 32: LoFTR full attention, key_cnt[b] = s for every sample.
+template <int D>
 __global__ void __launch_bounds__(fa::kThreads, 2)
 geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmV,
                       const __grid_constant__ CUtensorMap tmO, const __half* __restrict__ q16, int ldq,
-                      float* __restrict__ out, const int* __restrict__ anchor_cnt, int n_samples, int l, int heads,
+                      float* __restrict__ out, const int* __restrict__ key_cnt, int n_samples, int l, int heads,
                       float scale) {
   using namespace fa;
+  using C = Cfg<D>;
+  constexpr int kD = D, kKBytes = C::kKBytes, kVBytes = C::kVBytes, kColO = C::kColO, kColL = C::kColL, kColQ = C::kColQ;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sK = smem;
@@ -81,7 +96,7 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int q0 = blockIdx.x * kBQ, h = blockIdx.y, b = blockIdx.z;
   const int c = heads * kD;
-  const int cnt = anchor_cnt[b];
+  const int cnt = key_cnt[b];
   if (cnt <= 0) {   // no anchors: the layer is skipped for this sample (caller restores the features); emit zeros
     for (int e = threadIdx.x; e < kBQ * (kD / 4); e += blockDim.x) {
       const int r = e / (kD / 4), q = e - r * (kD / 4);
@@ -141,6 +156,7 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
     // (whole warp converged, one elected lane issues: operands stay in uniform registers - see conv_tc.cu)
     {
       constexpr uint32_t idesc = ptx::umma_idesc(0 /*f16*/, kBQ, 64);
+      constexpr uint32_t idesc_o = ptx::umma_idesc(0 /*f16*/, kBQ, kD);
       constexpr uint32_t idesc_l = ptx::umma_idesc(0 /*f16*/, kBQ, 16);
       ptx::mbar_wait(q_ready, 0);
       ptx::tc_fence_after();
@@ -159,7 +175,7 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
           const uint32_t b_lo = ptx::umma_desc_lo(sK0 + ks * kKBytes);
           if (ptx::elect_one()) {
 #pragma unroll
-            for (int k = 0; k < 4; ++k) ptx::umma_ts_f16_lo(tb + sb * 64, tb + kColQ + 8 * k, b_lo + 2 * k, ptx::kDescHiSw128, idesc, k ? 1u : 0u);
+            for (int k = 0; k < kD / 16; ++k) ptx::umma_ts_f16_lo(tb + sb * 64, tb + kColQ + 8 * k, b_lo + 2 * k, C::kKDescHi, idesc, k ? 1u : 0u);
             ptx::umma_commit_addr(bar_addr(&k_empty[ks]));
             ptx::umma_commit_addr(bar_addr(&s_full[sb]));
           }
@@ -175,7 +191,7 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
           const uint32_t acc0 = u > 0 ? 1u : 0u;
           if (ptx::elect_one()) {
 #pragma unroll
-            for (int k = 0; k < 4; ++k) ptx::umma_ts_f16_lo(tb + kColO, tb + pb * 64 + 8 * k, b_lo + 2 * k, ptx::kDescHiSw128, idesc, k ? 1u : acc0);
+            for (int k = 0; k < 4; ++k) ptx::umma_ts_f16_lo(tb + kColO, tb + pb * 64 + 8 * k, b_lo + 2 * k, ptx::kDescHiSw128, idesc_o, k ? 1u : acc0);
 #pragma unroll
             for (int k = 0; k < 4; ++k) ptx::umma_ts_f16_lo(tb + kColL, tb + pb * 64 + 8 * k, ones_lo + 2 * k, ptx::kDescHiSw128, idesc_l, k ? 1u : acc0);
             ptx::umma_commit_addr(bar_addr(&v_empty[vs]));
@@ -190,16 +206,17 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
     const int quad = warp & 3;                                     // TMEM lane quadrant (hardware: warp id % 4)
     const int row = quad * 32 + lane;                              // query row inside the CTA tile
     const uint32_t t_lane = tmem_base + (uint32_t(quad * 32) << 16);
-    {   // Q row -> tensor memory (A operand of every S MMA): 64 halves = 32 columns, two consecutive dims per column
-      uint4 qv[8];
+    {   // Q row -> tensor memory (A operand of every S MMA): D halves = D / 2 columns, two consecutive dims per column
+      uint4 qv[kD / 8];
 #pragma unroll
-      for (int j = 0; j < 8; ++j) qv[j] = make_uint4(0u, 0u, 0u, 0u);
+      for (int j = 0; j < kD / 8; ++j) qv[j] = make_uint4(0u, 0u, 0u, 0u);
       if (q0 + row < l) {
         const uint4* qg = reinterpret_cast<const uint4*>(q16 + ((int64_t)b * l + q0 + row) * ldq + h * kD);
 #pragma unroll
-        for (int j = 0; j < 8; ++j) qv[j] = __ldg(qg + j);
+        for (int j = 0; j < kD / 8; ++j) qv[j] = __ldg(qg + j);
       }
-      ptx::tmem_st_32x32(t_lane + kColQ, reinterpret_cast<const float*>(qv));
+      if constexpr (kD == 64) ptx::tmem_st_32x32(t_lane + kColQ, reinterpret_cast<const float*>(qv));
+      else ptx::tmem_st_32x16(t_lane + kColQ, reinterpret_cast<const float*>(qv));
       ptx::tmem_st_wait();
       ptx::tc_fence_before();
       __syncwarp();
@@ -244,7 +261,7 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
         ptx::tc_fence_after();
         float o[32];
 #pragma unroll
-        for (int hcol = 0; hcol < 2; ++hcol) {
+        for (int hcol = 0; hcol < kD / 32; ++hcol) {
           ptx::tmem_ld_32x32(t_lane + kColO + 32 * hcol, o);
           ptx::tmem_ld_wait();
 #pragma unroll
@@ -264,16 +281,16 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(&p_full[sb]);
     }
-    // epilogue: O / l -> two swizzled 32x32 fp32 boxes per warp (in the idle K / V ring) -> TMA store
+    // epilogue: O / l -> D / 32 swizzled 32x32 fp32 boxes per warp (in the idle K / V ring) -> TMA store
     ptx::mbar_wait(o_full, 0);
     ptx::tc_fence_after();
     float lsum[16];
     ptx::tmem_ld_32x16(t_lane + kColL, lsum);
     ptx::tmem_ld_wait();
     const float inv = 1.f / lsum[0];
-    uint8_t* wst = smem + (warp - 2) * 8192;
+    uint8_t* wst = smem + (warp - 2) * (kD / 32) * 4096;
 #pragma unroll
-    for (int hcol = 0; hcol < 2; ++hcol) {
+    for (int hcol = 0; hcol < kD / 32; ++hcol) {
       float o[32];
       ptx::tmem_ld_32x32(t_lane + kColO + 32 * hcol, o);
       ptx::tmem_ld_wait();
@@ -285,8 +302,8 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
     ptx::fence_proxy_async();
     __syncwarp();
     if (lane == 0) {
-      ptx::tma_store_3d(&tmO, wst, h * kD, q0 + quad * 32, b);
-      ptx::tma_store_3d(&tmO, wst + 4096, h * kD + 32, q0 + quad * 32, b);
+#pragma unroll
+      for (int hcol = 0; hcol < kD / 32; ++hcol) ptx::tma_store_3d(&tmO, wst + hcol * 4096, h * kD + 32 * hcol, q0 + quad * 32, b);
       ptx::bulk_commit();
       ptx::bulk_wait<0>();
     }
@@ -303,21 +320,66 @@ geo_flash_attn_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_cons
 
 using namespace gf;
 
+namespace gf {
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn encode_fn();
+}  // namespace gf
+
+// K tiles of head dim 32: dims {32, s_pad, heads * n} fp16, box {32 = 64 B, 64 keys, 1}, 64B swizzle
+static int make_k32_tmap(CUtensorMap* m, const void* kg, int64_t s_pad, int64_t batches) {
+  EncodeTiledFn enc = encode_fn();
+  if (!enc) return gf_set_error(GF_ERR_DRIVER, "gf_init() was not called");
+  cuuint64_t dims[3] = {32, (cuuint64_t)s_pad, (cuuint64_t)batches};
+  cuuint64_t strides[2] = {64, (cuuint64_t)s_pad * 64};
+  cuuint32_t box[3] = {32, (cuuint32_t)fa::kBK, 1};
+  cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(kg), dims, strides, box, estr,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return gf_set_error(GF_ERR_DRIVER, "cuTensorMapEncodeTiled(k32) failed");
+  return GF_OK;
+}
+
 // fp16 operands from gf_gather_anchor_kv_f16: q16 [n*l, heads*64] (head h at columns [h*64, h*64+64)),
 // kg [heads][n][s_pad][64], vt [heads][n][64][s_pad]; out fp32 [n*l, heads*64].
 extern "C" int gf_geo_self_attention_tc(const void* q16, int ldq, const void* kg, const void* vt, float* out, int n, int l,
                                         int heads, int dim, int s_pad, const int* anchor_cnt, gf_stream_t stream) {
+  using C = fa::Cfg<64>;
   const int c = heads * dim;
   if (n <= 0 || l <= 0 || heads <= 0 || dim != 64 || s_pad <= 0 || (s_pad % 8) || ldq < c || (ldq % 8))
     return gf_set_error(GF_ERR_ARG, "gf_geo_self_attention_tc: dim must be 64, s_pad % 8 == 0, ldq % 8 == 0");
   CUtensorMap tk, tv, to;
   int rc;
   if ((rc = make_tmap(&tk, kg, 2, dim, s_pad, (int64_t)heads * n, dim, (int64_t)s_pad * dim, fa::kBK))) return rc;
-  if ((rc = make_tmap(&tv, vt, 2, s_pad, dim, (int64_t)heads * n, s_pad, (int64_t)dim * s_pad, fa::kD))) return rc;
+  if ((rc = make_tmap(&tv, vt, 2, s_pad, dim, (int64_t)heads * n, s_pad, (int64_t)dim * s_pad, 64))) return rc;
   if ((rc = make_out_tmap(&to, out, c, l, n, c, (int64_t)l * c))) return rc;
-  GF_SMEM_OPTIN(geo_flash_attn_kernel, fa::kSmem);
-  geo_flash_attn_kernel<<<dim3(gf_cdiv(l, fa::kBQ), heads, n), fa::kThreads, fa::kSmem, (cudaStream_t)stream>>>(
+  GF_SMEM_OPTIN(geo_flash_attn_kernel<64>, C::kSmem);
+  geo_flash_attn_kernel<64><<<dim3(gf_cdiv(l, fa::kBQ), heads, n), fa::kThreads, C::kSmem, (cudaStream_t)stream>>>(
       tk, tv, to, (const __half*)q16, ldq, out, anchor_cnt, n, l, heads, 1.f / sqrtf((float)dim));
+  g_launches++;
+  GF_CHECK_LAUNCH();
+  return GF_OK;
+}
+
+// fp16 operands from gf_dense_kv_h16: q16 rows [n*l] with stride ldq (head h at columns [h*32, h*32+32)),
+// kg [heads][n][s_pad][32], vt [heads][n][32][s_pad] (zero for keys >= s); key_cnt [n] int32 on the device, every entry
+// s (written by gf_dense_kv_h16); out fp32 [n*l, heads*32].
+extern "C" int gf_full_attention_tc(const void* q16, int ldq, const void* kg, const void* vt, const int* key_cnt, float* out,
+                                    int n, int l, int s, int heads, int dim, int s_pad, gf_stream_t stream) {
+  using C = fa::Cfg<32>;
+  const int c = heads * dim;
+  if (n <= 0 || l <= 0 || s <= 0 || heads <= 0 || dim != 32 || s_pad < s || (s_pad % fa::kBK) || ldq < c || (ldq % 8))
+    return gf_set_error(GF_ERR_ARG, "gf_full_attention_tc: dim must be 32, s <= s_pad, s_pad % 64 == 0, ldq % 8 == 0");
+  CUtensorMap tk, tv, to;
+  int rc;
+  if ((rc = make_k32_tmap(&tk, kg, s_pad, (int64_t)heads * n))) return rc;
+  if ((rc = make_tmap(&tv, vt, 2, s_pad, dim, (int64_t)heads * n, s_pad, (int64_t)dim * s_pad, 32))) return rc;
+  if ((rc = make_out_tmap(&to, out, c, l, n, c, (int64_t)l * c))) return rc;
+  GF_SMEM_OPTIN(geo_flash_attn_kernel<32>, C::kSmem);
+  geo_flash_attn_kernel<32><<<dim3(gf_cdiv(l, fa::kBQ), heads, n), fa::kThreads, C::kSmem, (cudaStream_t)stream>>>(
+      tk, tv, to, (const __half*)q16, ldq, out, key_cnt, n, l, heads, 1.f / sqrtf((float)dim));
   g_launches++;
   GF_CHECK_LAUNCH();
   return GF_OK;

@@ -50,71 +50,79 @@ __global__ void geo_window_table_kernel(const float* __restrict__ hmat, const in
 // ---------------------------------------------------------------------------------------------
 // self attention against anchor tokens: flash-style online softmax, fp32 FFMA.
 // grid (ceil(l/64), heads, n); 256 threads as 16x16, each thread owns a 4x4 block of the 64x64 score tile
-// and a 4x4 block of the 64x64 output tile (dim == 64).
+// and a 4 x (D/16) block of the 64 x D output tile (head dim D = 64).
+// DENSE: every query attends to all s key rows of its sample (LoFTR full attention, linear_attention.py:54-85; D = 32
+// at the coarse level) instead of the anchor rows of its own image.
 // ---------------------------------------------------------------------------------------------
-constexpr int kSA = 64;          // queries per CTA == keys per tile == head dim
+constexpr int kSA = 64;          // queries per CTA == keys per tile
 constexpr int kSAPad = kSA + 4;
 
+template <int D>
+constexpr size_t self_attention_smem_bytes() { return (size_t)(kSA * D + D * kSAPad + kSA * (D + 4) + kSA * kSAPad) * sizeof(float); }
+
+template <int D, bool DENSE>
 __global__ void __launch_bounds__(256)
 geo_self_attention_kernel(const float* __restrict__ q, int ldq, const float* __restrict__ k, int ldk,
-                          const float* __restrict__ v, int ldv, float* __restrict__ out, int l, int heads,
+                          const float* __restrict__ v, int ldv, float* __restrict__ out, int l, int s, int heads,
                           const int* __restrict__ anchor_idx, const int* __restrict__ anchor_cnt, int anchor_cap,
                           float softmax_scale) {
+  constexpr int CW = D / 16;              // output columns per thread
+  constexpr int VP = D + 4;
   extern __shared__ float sh[];
-  float* Qs = sh;                         // [64][64]
-  float* Kt = Qs + kSA * kSA;             // [64 d][68 keys]
-  float* Vs = Kt + kSA * kSAPad;          // [64 keys][68]
-  float* Ps = Vs + kSA * kSAPad;          // [64 q][68]
+  float* Qs = sh;                         // [64][D]
+  float* Kt = Qs + kSA * D;               // [D][68 keys]
+  float* Vs = Kt + D * kSAPad;            // [64 keys][D + 4]
+  float* Ps = Vs + kSA * VP;              // [64 q][68]
   const int n = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * kSA;
-  const int cnt = anchor_cnt[n];
-  const int c = heads * kSA;
+  const int cnt = DENSE ? s : anchor_cnt[n];
+  const int c = heads * D;
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
   if (cnt == 0) {
-    for (int e = tid; e < kSA * kSA; e += 256) {
-      const int r = e >> 6, d = e & 63;
-      if (q0 + r < l) out[((int64_t)n * l + q0 + r) * c + h * kSA + d] = 0.f;
+    for (int e = tid; e < kSA * D; e += 256) {
+      const int r = e / D, d = e % D;
+      if (q0 + r < l) out[((int64_t)n * l + q0 + r) * c + h * D + d] = 0.f;
     }
     return;
   }
-  for (int e = tid; e < kSA * kSA; e += 256) {
-    const int r = e >> 6, d = e & 63;
-    Qs[e] = (q0 + r < l) ? q[((int64_t)n * l + q0 + r) * ldq + h * kSA + d] : 0.f;
+  for (int e = tid; e < kSA * D; e += 256) {
+    const int r = e / D, d = e % D;
+    Qs[e] = (q0 + r < l) ? q[((int64_t)n * l + q0 + r) * ldq + h * D + d] : 0.f;
   }
-  float m_run[4], l_run[4], o[4][4];
+  float m_run[4], l_run[4], o[4][CW];
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     m_run[i] = -INFINITY; l_run[i] = 0.f;
 #pragma unroll
-    for (int j = 0; j < 4; ++j) o[i][j] = 0.f;
+    for (int j = 0; j < CW; ++j) o[i][j] = 0.f;
   }
-  const int* aidx = anchor_idx + (int64_t)n * anchor_cap;
+  const int* aidx = DENSE ? nullptr : anchor_idx + (int64_t)n * anchor_cap;
   for (int k0 = 0; k0 < cnt; k0 += kSA) {
     __syncthreads();   // previous tile fully consumed (also covers the Qs fill on the first iteration)
-    for (int e = tid; e < kSA * kSA; e += 256) {
-      const int r = e >> 6, d = e & 63;
+    for (int e = tid; e < kSA * D; e += 256) {
+      const int r = e / D, d = e % D;
       float kv = 0.f, vv = 0.f;
       if (k0 + r < cnt) {
-        const int64_t tok = (int64_t)n * l + aidx[k0 + r];
-        kv = k[tok * ldk + h * kSA + d];
-        vv = v[tok * ldv + h * kSA + d];
+        const int64_t tok = DENSE ? (int64_t)n * s + k0 + r : (int64_t)n * l + aidx[k0 + r];
+        kv = k[tok * ldk + h * D + d];
+        vv = v[tok * ldv + h * D + d];
       }
       Kt[d * kSAPad + r] = kv;
-      Vs[r * kSAPad + d] = vv;
+      Vs[r * VP + d] = vv;
     }
     __syncthreads();
-    float s[4][4];
+    float s_[4][4];
 #pragma unroll
     for (int i = 0; i < 4; ++i)
 #pragma unroll
-      for (int j = 0; j < 4; ++j) s[i][j] = 0.f;
+      for (int j = 0; j < 4; ++j) s_[i][j] = 0.f;
 #pragma unroll 8
-    for (int d = 0; d < kSA; ++d) {
+    for (int d = 0; d < D; ++d) {
       const float4 kk = *reinterpret_cast<const float4*>(&Kt[d * kSAPad + 4 * tx]);
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
-        const float qv = Qs[(4 * ty + i) * kSA + d];
-        s[i][0] = fmaf(qv, kk.x, s[i][0]); s[i][1] = fmaf(qv, kk.y, s[i][1]);
-        s[i][2] = fmaf(qv, kk.z, s[i][2]); s[i][3] = fmaf(qv, kk.w, s[i][3]);
+        const float qv = Qs[(4 * ty + i) * D + d];
+        s_[i][0] = fmaf(qv, kk.x, s_[i][0]); s_[i][1] = fmaf(qv, kk.y, s_[i][1]);
+        s_[i][2] = fmaf(qv, kk.z, s_[i][2]); s_[i][3] = fmaf(qv, kk.w, s_[i][3]);
       }
     }
     float alpha[4];
@@ -123,8 +131,8 @@ geo_self_attention_kernel(const float* __restrict__ q, int ldq, const float* __r
       float mx = -INFINITY;
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
-        s[i][j] = (k0 + 4 * tx + j < cnt) ? s[i][j] * softmax_scale : -INFINITY;
-        mx = fmaxf(mx, s[i][j]);
+        s_[i][j] = (k0 + 4 * tx + j < cnt) ? s_[i][j] * softmax_scale : -INFINITY;
+        mx = fmaxf(mx, s_[i][j]);
       }
 #pragma unroll
       for (int off = 8; off > 0; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
@@ -132,24 +140,31 @@ geo_self_attention_kernel(const float* __restrict__ q, int ldq, const float* __r
       alpha[i] = expf(m_run[i] - m_new);
       float rs = 0.f;
 #pragma unroll
-      for (int j = 0; j < 4; ++j) { s[i][j] = expf(s[i][j] - m_new); rs += s[i][j]; }
+      for (int j = 0; j < 4; ++j) { s_[i][j] = expf(s_[i][j] - m_new); rs += s_[i][j]; }
 #pragma unroll
       for (int off = 8; off > 0; off >>= 1) rs += __shfl_xor_sync(0xffffffffu, rs, off);
       l_run[i] = l_run[i] * alpha[i] + rs;
       m_run[i] = m_new;
-      *reinterpret_cast<float4*>(&Ps[(4 * ty + i) * kSAPad + 4 * tx]) = make_float4(s[i][0], s[i][1], s[i][2], s[i][3]);
+      *reinterpret_cast<float4*>(&Ps[(4 * ty + i) * kSAPad + 4 * tx]) = make_float4(s_[i][0], s_[i][1], s_[i][2], s_[i][3]);
 #pragma unroll
-      for (int j = 0; j < 4; ++j) o[i][j] *= alpha[i];
+      for (int j = 0; j < CW; ++j) o[i][j] *= alpha[i];
     }
     __syncthreads();
 #pragma unroll 8
     for (int kk = 0; kk < kSA; ++kk) {
-      const float4 vv = *reinterpret_cast<const float4*>(&Vs[kk * kSAPad + 4 * tx]);
+      float vv[CW];
+      if constexpr (CW == 4) {
+        const float4 t = *reinterpret_cast<const float4*>(&Vs[kk * VP + 4 * tx]);
+        vv[0] = t.x; vv[1] = t.y; vv[2] = t.z; vv[3] = t.w;
+      } else {
+        const float2 t = *reinterpret_cast<const float2*>(&Vs[kk * VP + 2 * tx]);
+        vv[0] = t.x; vv[1] = t.y;
+      }
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
         const float pv = Ps[(4 * ty + i) * kSAPad + kk];
-        o[i][0] = fmaf(pv, vv.x, o[i][0]); o[i][1] = fmaf(pv, vv.y, o[i][1]);
-        o[i][2] = fmaf(pv, vv.z, o[i][2]); o[i][3] = fmaf(pv, vv.w, o[i][3]);
+#pragma unroll
+        for (int j = 0; j < CW; ++j) o[i][j] = fmaf(pv, vv[j], o[i][j]);
       }
     }
   }
@@ -158,8 +173,9 @@ geo_self_attention_kernel(const float* __restrict__ q, int ldq, const float* __r
     const int r = q0 + 4 * ty + i;
     if (r < l) {
       const float inv = 1.f / l_run[i];
-      *reinterpret_cast<float4*>(&out[((int64_t)n * l + r) * c + h * kSA + 4 * tx]) =
-          make_float4(o[i][0] * inv, o[i][1] * inv, o[i][2] * inv, o[i][3] * inv);
+      float* dst = &out[((int64_t)n * l + r) * c + h * D + CW * tx];
+      if constexpr (CW == 4) *reinterpret_cast<float4*>(dst) = make_float4(o[i][0] * inv, o[i][1] * inv, o[i][2] * inv, o[i][3] * inv);
+      else *reinterpret_cast<float2*>(dst) = make_float2(o[i][0] * inv, o[i][1] * inv);
     }
   }
 }
@@ -310,33 +326,36 @@ __global__ void gather_anchor_kv_f16_kernel(const float* __restrict__ q, int ldq
 
 // Same gather from fp16 K / V rows (the OUT16 projection): kg rows are copied as 16-byte chunks, the V tile of 64
 // anchors is transposed through shared memory so that vt rows leave as 16-byte vectors too.  grid (s_pad / 64, n),
-// 256 threads; heads * dim == 256, dim == 64.
+// 256 threads; heads * D == 256.  DENSE: key j of sample b is row b * s + j of K / V (all s rows, no anchor list), and
+// block (0, b) also writes key_cnt[b] = s for the flash kernel.
+template <int D, bool DENSE>
 __global__ void __launch_bounds__(256)
 gather_anchor_kv_h16_kernel(const __half* __restrict__ k, int ldk, const __half* __restrict__ v, int ldv, int n, int l,
                             const int* __restrict__ anchor_idx, const int* __restrict__ anchor_cnt, int anchor_cap,
-                            int s_pad, __half* __restrict__ kg, __half* __restrict__ vt) {
-  constexpr int C = 256, D = 64, PITCH = C + 8;
+                            int s_pad, __half* __restrict__ kg, __half* __restrict__ vt, int* __restrict__ key_cnt) {
+  constexpr int C = 256, PITCH = C + 8, CH = D / 8;           // CH: 16-byte chunks per head row
   __shared__ __align__(16) __half vs[64 * PITCH];
   const int b = blockIdx.y, s0 = blockIdx.x * 64, t = threadIdx.x;
-  const int cnt = anchor_cnt[b];
+  const int cnt = DENSE ? l : anchor_cnt[b];                  // dense: l is the key count s of every sample
+  if (DENSE && blockIdx.x == 0 && t == 0) key_cnt[b] = cnt;
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const int e = t + 256 * i, r = e >> 5, q = e & 31;       // anchor row r of the tile, 16-byte chunk q of its 512 B
     const int s = s0 + r;
     uint4 kq = make_uint4(0u, 0u, 0u, 0u), vq = kq;
     if (s < cnt) {
-      const int64_t tok = (int64_t)b * l + anchor_idx[(int64_t)b * anchor_cap + s];
+      const int64_t tok = DENSE ? (int64_t)b * l + s : (int64_t)b * l + anchor_idx[(int64_t)b * anchor_cap + s];
       kq = __ldg(reinterpret_cast<const uint4*>(k + tok * ldk) + q);
       vq = __ldg(reinterpret_cast<const uint4*>(v + tok * ldv) + q);
     }
     if (s < s_pad) {
-      const int h = q >> 3;
-      *reinterpret_cast<uint4*>(kg + (((int64_t)h * n + b) * s_pad + s) * D + (q & 7) * 8) = kq;
+      const int h = q / CH;
+      *reinterpret_cast<uint4*>(kg + (((int64_t)h * n + b) * s_pad + s) * D + (q % CH) * 8) = kq;
     }
     *reinterpret_cast<uint4*>(vs + r * PITCH + q * 8) = vq;
   }
   __syncthreads();
-  const int h = t >> 6, d = t & 63;                           // thread == channel
+  const int h = t / D, d = t % D;                             // thread == channel
   __half* dst = vt + (((int64_t)h * n + b) * D + d) * s_pad + s0;
 #pragma unroll
   for (int g8 = 0; g8 < 8; ++g8) {
@@ -412,10 +431,10 @@ extern "C" int gf_geo_self_attention(const float* q, int ldq, const float* k, in
                                      float* out, int n, int l, int heads, int dim, const int* anchor_idx,
                                      const int* anchor_cnt, int anchor_cap, gf_stream_t stream) {
   if (n <= 0 || l <= 0 || heads <= 0 || dim != 64) return gf_set_error(GF_ERR_ARG, "gf_geo_self_attention: dim must be 64");
-  const size_t smem = (size_t)(kSA * kSA + 3 * kSA * kSAPad) * sizeof(float);
-  GF_SMEM_OPTIN(geo_self_attention_kernel, smem);
-  geo_self_attention_kernel<<<dim3(gf_cdiv(l, kSA), heads, n), 256, smem, STREAM>>>(
-      q, ldq, k, ldk, v, ldv, out, l, heads, anchor_idx, anchor_cnt, anchor_cap, 1.f / sqrtf((float)dim));
+  constexpr size_t smem = self_attention_smem_bytes<64>();
+  GF_SMEM_OPTIN((geo_self_attention_kernel<64, false>), smem);
+  geo_self_attention_kernel<64, false><<<dim3(gf_cdiv(l, kSA), heads, n), 256, smem, STREAM>>>(
+      q, ldq, k, ldk, v, ldv, out, l, l, heads, anchor_idx, anchor_cnt, anchor_cap, 1.f / sqrtf((float)dim));
   g_launches++;
   GF_CHECK_LAUNCH();
   return GF_OK;
@@ -476,9 +495,36 @@ extern "C" int gf_gather_anchor_kv_h16(const void* k, int ldk, const void* v, in
                                        void* vt, gf_stream_t stream) {
   if (n <= 0 || l <= 0 || heads * dim != 256 || dim != 64 || s_pad <= 0 || (s_pad % 8) || (ldk % 8) || (ldv % 8))
     return gf_set_error(GF_ERR_ARG, "gf_gather_anchor_kv_h16: needs 4 heads of dim 64, s_pad % 8 == 0, 16-byte aligned rows");
-  gather_anchor_kv_h16_kernel<<<dim3(gf_cdiv(s_pad, 64), n), 256, 0, STREAM>>>((const __half*)k, ldk, (const __half*)v, ldv, n, l,
-                                                                             anchor_idx, anchor_cnt, anchor_cap, s_pad,
-                                                                             (__half*)kg, (__half*)vt);
+  gather_anchor_kv_h16_kernel<64, false><<<dim3(gf_cdiv(s_pad, 64), n), 256, 0, STREAM>>>(
+      (const __half*)k, ldk, (const __half*)v, ldv, n, l, anchor_idx, anchor_cnt, anchor_cap, s_pad, (__half*)kg, (__half*)vt,
+      nullptr);
+  g_launches++;
+  GF_CHECK_LAUNCH();
+  return GF_OK;
+}
+
+// LoFTR full attention (linear_attention.py:54-85) over dense keys, fp32 FFMA: out[n*l, heads*32] from the query rows
+// q [n*l] and the key / value rows k, v [n*s] (row strides ldq / ldk / ldv floats); scale 1/sqrt(32).
+extern "C" int gf_full_attention(const float* q, int ldq, const float* k, int ldk, const float* v, int ldv, float* out,
+                                 int n, int l, int s, int heads, int dim, gf_stream_t stream) {
+  if (n <= 0 || l <= 0 || s <= 0 || heads <= 0 || dim != 32) return gf_set_error(GF_ERR_ARG, "gf_full_attention: dim must be 32");
+  constexpr size_t smem = self_attention_smem_bytes<32>();
+  GF_SMEM_OPTIN((geo_self_attention_kernel<32, true>), smem);
+  geo_self_attention_kernel<32, true><<<dim3(gf_cdiv(l, kSA), heads, n), 256, smem, STREAM>>>(
+      q, ldq, k, ldk, v, ldv, out, l, s, heads, nullptr, nullptr, 0, 1.f / sqrtf((float)dim));
+  g_launches++;
+  GF_CHECK_LAUNCH();
+  return GF_OK;
+}
+
+// Dense K / V^T tiles of gf_full_attention_tc from fp16 K / V rows [n*s] (8 heads of dim 32):
+// kg[h][n][s_pad][32], vt[h][n][32][s_pad] (zero for keys >= s) and key_cnt[n] = s.
+extern "C" int gf_dense_kv_h16(const void* k, int ldk, const void* v, int ldv, int n, int s, int heads, int dim, int s_pad,
+                               void* kg, void* vt, int* key_cnt, gf_stream_t stream) {
+  if (n <= 0 || s <= 0 || heads * dim != 256 || dim != 32 || s_pad < s || (s_pad % 64) || (ldk % 8) || (ldv % 8))
+    return gf_set_error(GF_ERR_ARG, "gf_dense_kv_h16: needs 8 heads of dim 32, s <= s_pad, s_pad % 64 == 0, 16-byte rows");
+  gather_anchor_kv_h16_kernel<32, true><<<dim3(s_pad / 64, n), 256, 0, STREAM>>>(
+      (const __half*)k, ldk, (const __half*)v, ldv, n, s, nullptr, nullptr, 0, s_pad, (__half*)kg, (__half*)vt, key_cnt);
   g_launches++;
   GF_CHECK_LAUNCH();
   return GF_OK;

@@ -132,6 +132,7 @@ __device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t adesc, uint64_t b
 // changes between the MMAs of a tile, so the per-MMA arithmetic is one 32-bit add that stays in a uniform register.
 // Call from a CONVERGED warp under `if (elect_one())` (see conv_tc.cu for why).
 constexpr uint32_t kDescHiSw128 = (1024u >> 4) | (1u << 14) | (2u << 29);     // SBO 1024 B, version 1, SWIZZLE_128B
+constexpr uint32_t kDescHiSw64 = (512u >> 4) | (1u << 14) | (4u << 29);       // SBO 512 B, version 1, SWIZZLE_64B
 constexpr uint32_t kDescHiSw32 = (256u >> 4) | (1u << 14) | (6u << 29);       // SBO 256 B, version 1, SWIZZLE_32B
 __device__ __forceinline__ uint32_t umma_desc_lo(uint32_t smem_byte_addr) {
   return ((smem_byte_addr >> 4) & 0x3FFFu) | (1u << 16);

@@ -282,12 +282,39 @@ def _post_attention(lw: dict, x2d: torch.Tensor, msg: torch.Tensor, act: int, ou
     return ops.linear(h, lw["w2_16"] if h16 else lw["w2"], epi=EPI_LN, gamma=lw["n2w"], beta=lw["n2b"], residual=x2d, out=out)
 
 
+def _full_attention_layer(lw: dict, x: torch.Tensor, src: torch.Tensor, heads: int, out: Optional[torch.Tensor]):
+    """LoFTR encoder layer with `attention: 'full'` (linear_attention.py:54-85): plain Q / K / V projections (no elu+1
+    epilogue), softmax attention over all S source tokens, then the same merge / norm / MLP as the linear route.
+    Product mode stores Q|K|V in fp16 for the tcgen05 flash kernel (heads x 32); otherwise fp32 for the FFMA kernel."""
+    n, l, c = x.shape
+    s = src.shape[1]
+    d = c // heads
+    x2d = x.reshape(n * l, c)
+    a16 = ops.act16() and ops._ATTN_IMPL != "ref" and (c, d) == (256, 32)
+    if x is src:
+        qkv = ops.linear(x2d, lw["wqkv"], out_f16=a16)
+        q, k, v, ldq, ldk = qkv, qkv[:, c:], qkv[:, 2 * c:], 3 * c, 3 * c
+    else:
+        q = ops.linear(x2d, lw["wq"], out_f16=a16)
+        kv = ops.linear(src.reshape(n * s, c), lw["wkv"], out_f16=a16)
+        k, v, ldq, ldk = kv, kv[:, c:], c, 2 * c
+    msg = ops.full_attention(q, ldq, k, ldk, v, ldk, n, l, s, heads, d)
+    return _post_attention(lw, x2d, msg, EPI_RELU, None if out is None else out.view(n * l, c)).view(n, l, c)
+
+
 def loftr_layer(lw: dict, x: torch.Tensor, src: torch.Tensor, heads: int, out: Optional[torch.Tensor] = None,
-                q_mask: Optional[torch.Tensor] = None, kv_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """LoFTR encoder layer with linear attention; x [n,L,C], src [n,S,C] -> [n,L,C] (written into `out` if given).
-    q_mask [n,L] / kv_mask [n,S] (uint8, 0 = padded token; optional): the feature-mapped Q / K rows and the value rows of
-    padded tokens are cleared before the attention (linear_attention.py:37-43); the sequence length S that scales the
-    values keeps counting them (linear_attention.py:45)."""
+                q_mask: Optional[torch.Tensor] = None, kv_mask: Optional[torch.Tensor] = None,
+                attention: str = "linear") -> torch.Tensor:
+    """LoFTR encoder layer with linear (default) or full softmax attention; x [n,L,C], src [n,S,C] -> [n,L,C] (written
+    into `out` if given).  q_mask [n,L] / kv_mask [n,S] (uint8, 0 = padded token; optional; linear attention only): the
+    feature-mapped Q / K rows and the value rows of padded tokens are cleared before the attention
+    (linear_attention.py:37-43); the sequence length S that scales the values keeps counting them
+    (linear_attention.py:45)."""
+    if attention == "full":
+        if q_mask is not None or kv_mask is not None:
+            raise NotImplementedError("full attention with padding masks is not supported")
+        return _full_attention_layer(lw, x, src, heads, out)
+    assert attention == "linear", attention
     n, l, c = x.shape
     s = src.shape[1]
     d = c // heads
@@ -316,8 +343,10 @@ def loftr_layer(lw: dict, x: torch.Tensor, src: torch.Tensor, heads: int, out: O
 
 
 def coarse_transformer(pw: PackedWeights, x0: torch.Tensor, x1: torch.Tensor, names, heads: int,
-                       mask0: Optional[torch.Tensor] = None, mask1: Optional[torch.Tensor] = None):
+                       mask0: Optional[torch.Tensor] = None, mask1: Optional[torch.Tensor] = None,
+                       attention: str = "linear"):
     """loftr_module/transformer.py:82-104.  Same-size pairs run both images as one 2n-sample batch.
+    attention: 'linear' or 'full' (the config's coarse.attention; every layer uses the same kind).
     mask0 [n,L] / mask1 [n,S] (uint8 token masks from ops.token_mask, both or neither): self layers mask queries and
     sources with the image's own mask, cross layers the queries with their own and the sources with the other image's
     (transformer.py:95-100)."""
@@ -333,27 +362,42 @@ def coarse_transformer(pw: PackedWeights, x0: torch.Tensor, x1: torch.Tensor, na
     for lw, name in zip(pw.coarse, names):
         if name == "self":
             if same:
-                X = loftr_layer(lw, X, X, heads, q_mask=mm, kv_mask=mm)
+                X = loftr_layer(lw, X, X, heads, q_mask=mm, kv_mask=mm, attention=attention)
                 x0, x1 = X[:n], X[n:]
             else:
-                x0 = loftr_layer(lw, x0, x0, heads, q_mask=mask0, kv_mask=mask0)
-                x1 = loftr_layer(lw, x1, x1, heads, q_mask=mask1, kv_mask=mask1)
+                x0 = loftr_layer(lw, x0, x0, heads, q_mask=mask0, kv_mask=mask0, attention=attention)
+                x1 = loftr_layer(lw, x1, x1, heads, q_mask=mask1, kv_mask=mask1, attention=attention)
         elif same:                                    # both results land in the halves of one fresh 2n-sample buffer
             Xn = torch.empty_like(X)
-            y0 = loftr_layer(lw, x0, x1, heads, out=Xn[:n], q_mask=mask0, kv_mask=mask1)
-            loftr_layer(lw, x1, y0, heads, out=Xn[n:], q_mask=mask1, kv_mask=mask0)   # sees the UPDATED feat0 (transformer.py:99-100)
+            y0 = loftr_layer(lw, x0, x1, heads, out=Xn[:n], q_mask=mask0, kv_mask=mask1, attention=attention)
+            loftr_layer(lw, x1, y0, heads, out=Xn[n:], q_mask=mask1, kv_mask=mask0, attention=attention)   # sees the UPDATED feat0 (transformer.py:99-100)
             X = Xn
             x0, x1 = X[:n], X[n:]
         else:
-            y0 = loftr_layer(lw, x0, x1, heads, q_mask=mask0, kv_mask=mask1)
-            x0, x1 = y0, loftr_layer(lw, x1, y0, heads, q_mask=mask1, kv_mask=mask0)
+            y0 = loftr_layer(lw, x0, x1, heads, q_mask=mask0, kv_mask=mask1, attention=attention)
+            x0, x1 = y0, loftr_layer(lw, x1, y0, heads, q_mask=mask1, kv_mask=mask0, attention=attention)
     return x0, x1
 
 
-def fine_layer(lw: dict, x: torch.Tensor, src: torch.Tensor, heads: int) -> torch.Tensor:
-    """LoFTR layer at the fine level: x/src [m, 25, 128]; one CTA per window for the attention."""
+def fine_layer(lw: dict, x: torch.Tensor, src: torch.Tensor, heads: int, attention: str = "linear") -> torch.Tensor:
+    """LoFTR layer at the fine level: x/src [m, 25, 128]; one CTA per window for the linear attention, one warp per
+    (window, head) for the full one (attention='full', which always takes the per-op path: the fused layer kernel is
+    linear-only)."""
     m, t, c = x.shape
     d = c // heads
+    if attention == "full":
+        x2d = x.reshape(m * t, c)
+        a16 = ops.act16() and ops._ATTN_IMPL != "ref" and d == 16
+        if x is src:
+            qkv = ops.linear(x2d, lw["wqkv"], out_f16=a16)
+            q, k, v, ldq, ldk = qkv, qkv[:, c:], qkv[:, 2 * c:], 3 * c, 3 * c
+        else:
+            q = ops.linear(x2d, lw["wq"], out_f16=a16)
+            kv = ops.linear(src.reshape(m * t, c), lw["wkv"], out_f16=a16)
+            k, v, ldq, ldk = kv, kv[:, c:], c, 2 * c
+        msg = ops.full_attention_window(q, ldq, k, ldk, v, ldk, m, t, heads, d)
+        return _post_attention(lw, x2d, msg, EPI_RELU).view(m, t, c)
+    assert attention == "linear", attention
     if FUSED_FINE_LAYER and ops.act16() and (t, c, heads) == (25, 128, 8) and "wpack" in lw:
         return ops.fine_layer_fused(x.contiguous(), src.contiguous(), lw["wpack"], lw["n1w"], lw["n1b"], lw["n2w"], lw["n2b"])
     x2d = x.reshape(m * t, c)
@@ -538,7 +582,7 @@ def geo_module(pw: PackedWeights, x0: torch.Tensor, x1: torch.Tensor, first: dic
 # --------------------------------------------------------------------------------------------
 def fine_stage(pw: PackedWeights, fine0: torch.Tensor, fine1: torch.Tensor, g0: torch.Tensor, g1: torch.Tensor,
                m2: dict, hw0_i, hw0_c, hw1_c, hw0_f, window: int, heads: int, names, temperature: float, thr: float,
-               want_matrix: bool):
+               want_matrix: bool, attention: str = "linear"):
     b_ids, i_ids, j_ids = m2["b_ids"], m2["i_ids"], m2["j_ids"]
     m = b_ids.shape[0]
     dev = fine0.device
@@ -561,11 +605,11 @@ def fine_stage(pw: PackedWeights, fine0: torch.Tensor, fine1: torch.Tensor, g0: 
     f0, f1 = X[:m], X[m:]
     for lw, name in zip(pw.fine, names):
         if name == "self":
-            X = fine_layer(lw, X, X, heads)
+            X = fine_layer(lw, X, X, heads, attention)
             f0, f1 = X[:m], X[m:]
         else:
-            y0 = fine_layer(lw, f0, f1, heads)
-            y1 = fine_layer(lw, f1, y0, heads)
+            y0 = fine_layer(lw, f0, f1, heads, attention)
+            y1 = fine_layer(lw, f1, y0, heads, attention)
             f0, f1 = y0, y1
     coarse_scale = hw0_i[0] / hw0_c[0]
     c2f = hw0_f[0] / hw0_c[0]

@@ -88,6 +88,16 @@ class _GeoModule(nn.Module):
 _BACKBONE_DTYPES = {"f16": torch.float16, "fp32": torch.float32}
 
 
+def _attention_kinds(cfg) -> tuple:
+    """(coarse, fine) attention of the LoFTR config: 'linear' (LinearAttention) or 'full' (FullAttention), read as
+    loftr_module/transformer.py:22 does; anything else is refused."""
+    kinds = tuple(cfg[level].get("attention", "linear") for level in ("coarse", "fine"))
+    for level, kind in zip(("coarse", "fine"), kinds):
+        if kind not in ("linear", "full"):
+            raise ValueError(f"geoformer_b200.GeoFormer: {level}.attention must be 'linear' or 'full', got {kind!r}")
+    return kinds
+
+
 class GeoFormer(nn.Module):
     def __init__(self, loftr_config, geoformer_cfg=default_cfg):
         super().__init__()
@@ -116,6 +126,13 @@ class GeoFormer(nn.Module):
         if loftr_config["coarse"].get("temp_bug_fix", False):
             # position_encoding.py:26-28: only the (default) bug-compatible table is implemented
             raise NotImplementedError("geoformer_b200.GeoFormer: coarse.temp_bug_fix=True is not supported")
+        _attention_kinds(loftr_config)
+        if loftr_config["match_coarse"].get("match_type", "dual_softmax") != "dual_softmax":
+            # sinkhorn (coarse_matching.py:100-108) needs a bin_score parameter that the checkpoint schema does not hold
+            raise NotImplementedError("geoformer_b200.GeoFormer: match_coarse.match_type must be 'dual_softmax'")
+        if not loftr_config.get("fine_concat_coarse_feat", True):
+            # fine_preprocess.py:58-72: only the merge_feat route (coarse feature concatenated to the windows) is built
+            raise NotImplementedError("geoformer_b200.GeoFormer: fine_concat_coarse_feat=False is not supported")
 
     # ---- parameter bookkeeping -----------------------------------------------------------------
     def load_state_dict(self, state_dict, *args, **kwargs):
@@ -177,6 +194,10 @@ class GeoFormer(nn.Module):
             # only exist in the training collations; ignoring them would silently change the result.
             if data.get(k) is not None:
                 raise NotImplementedError(f"geoformer_b200.GeoFormer: data[{k!r}] is not supported (training-only key)")
+        if data.get("mask0") is not None and _attention_kinds(self.config)[0] == "full":
+            # FullAttention (linear_attention.py:75-77) fills masked logits with -inf: a fully padded query row is a softmax
+            # over -inf only (NaN), which the next layer spreads into valid rows; there is no result to reproduce
+            raise NotImplementedError("geoformer_b200.GeoFormer: coarse.attention='full' with padding masks is not supported")
         if not img0.is_cuda:
             raise RuntimeError("geoformer_b200.GeoFormer runs on CUDA (sm_100a) only; there is no CPU fallback")
         with torch.cuda.device(img0.device):       # kernels launch on the tensors' device and its current stream
@@ -188,6 +209,7 @@ class GeoFormer(nn.Module):
     def _forward(self, data, img0, img1):
         pw = self._weights(img0.device)
         cfg, gcfg = self.config, self.geo_cfg
+        att_c, att_f = _attention_kinds(cfg)
         n = img0.shape[0]
         hw0_i, hw1_i = tuple(img0.shape[2:]), tuple(img1.shape[2:])
         data.update({"bs": torch.tensor(n), "hw0_i": torch.tensor(hw0_i), "hw1_i": torch.tensor(hw1_i)})
@@ -216,7 +238,8 @@ class GeoFormer(nn.Module):
         with R("stage:coarse_transformer"):
             x0 = ops.add_posenc(c0.reshape(n, -1, dc), pw.pos_table(dc, *hw0_c))
             x1 = ops.add_posenc(c1.reshape(n, -1, dc), pw.pos_table(dc, *hw1_c))
-            t0, t1 = engine.coarse_transformer(pw, x0, x1, cfg["coarse"]["layer_names"], cfg["coarse"]["nhead"], mk0, mk1)
+            t0, t1 = engine.coarse_transformer(pw, x0, x1, cfg["coarse"]["layer_names"], cfg["coarse"]["nhead"], mk0, mk1,
+                                               attention=att_c)
 
         # 3. coarse matching -> geo module -> coarse matching (full_model.py:87-90)
         thr = cfg["match_coarse"]["thr"]
@@ -247,7 +270,8 @@ class GeoFormer(nn.Module):
             with R("stage:fine"):
                 out, fmat, fstages = engine.fine_stage(pw, f0, f1, g0, g1, m2, hw0_i, hw0_c, hw1_c, hw0_f, w,
                                                        cfg["fine"]["nhead"], cfg["fine"]["layer_names"],
-                                                       gcfg["fine_temperature"], gcfg["fine_thr"], self.materialize)
+                                                       gcfg["fine_temperature"], gcfg["fine_thr"], self.materialize,
+                                                       attention=att_f)
             data.update(out)
             if self.materialize:
                 data["fine_matrix"] = fmat

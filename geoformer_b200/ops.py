@@ -348,6 +348,42 @@ def linattn_window(q: torch.Tensor, ldq: int, k: torch.Tensor, ldk: int, v: torc
     return out
 
 
+def full_attention(q: torch.Tensor, ldq: int, k: torch.Tensor, ldk: int, v: torch.Tensor, ldv: int, n: int, l: int, s: int,
+                   heads: int, dim: int) -> torch.Tensor:
+    """LoFTR full attention (linear_attention.py:54-85): softmax(Q K^T / sqrt(dim)) V of every query row against all s key
+    rows of its sample; q rows [n*l], k / v rows [n*s] (views with row strides ldq / ldk / ldv elements).  fp16 Q|K|V: the
+    tcgen05 flash kernel (gf_dense_kv_h16 + gf_full_attention_tc, dim 32, heads*dim == 256); fp32: the FFMA kernel
+    (accurate mode).  Returns the fp32 message [n*l, heads*dim]."""
+    assert q.dtype == k.dtype == v.dtype
+    dev = q.device
+    out = torch.empty((n * l, heads * dim), device=dev, dtype=torch.float32)
+    if q.dtype == torch.float16:
+        s_pad = (s + 63) // 64 * 64
+        kg = torch.empty((heads, n, s_pad, dim), device=dev, dtype=torch.float16)
+        vt = torch.empty((heads, n, dim, s_pad), device=dev, dtype=torch.float16)
+        cnt = torch.empty(n, device=dev, dtype=torch.int32)
+        _call("gf_dense_kv_h16", k.data_ptr(), ldk, v.data_ptr(), ldv, n, s, heads, dim, s_pad, kg.data_ptr(), vt.data_ptr(),
+              cnt.data_ptr(), _stream())
+        _call("gf_full_attention_tc", q.data_ptr(), ldq, kg.data_ptr(), vt.data_ptr(), cnt.data_ptr(), out.data_ptr(), n, l,
+              s, heads, dim, s_pad, _stream())
+        return out
+    _chk(q)
+    _call("gf_full_attention", q.data_ptr(), ldq, k.data_ptr(), ldk, v.data_ptr(), ldv, out.data_ptr(), n, l, s, heads, dim,
+          _stream())
+    return out
+
+
+def full_attention_window(q: torch.Tensor, ldq: int, k: torch.Tensor, ldk: int, v: torch.Tensor, ldv: int, n_windows: int,
+                          tokens: int, heads: int, dim: int) -> torch.Tensor:
+    """Full attention inside fine-level windows: window m's `tokens` query rows against window m's key / value rows.
+    fp16 or fp32 Q|K|V; returns the fp32 message [n_windows*tokens, heads*dim]."""
+    assert q.dtype == k.dtype == v.dtype
+    out = torch.empty((n_windows * tokens, heads * dim), device=q.device, dtype=torch.float32)
+    _call("gf_full_attention_window" + ("_f16" if q.dtype == torch.float16 else ""), q.data_ptr(), ldq, k.data_ptr(), ldk,
+          v.data_ptr(), ldv, out.data_ptr(), n_windows, tokens, heads, dim, _stream())
+    return out
+
+
 def fine_layer_fused(x: torch.Tensor, src: torch.Tensor, wpack: torch.Tensor, n1w, n1b, n2w, n2b) -> torch.Tensor:
     """One fine-level LoFTR layer in a single kernel (csrc/fine_layer.cu).  x/src [m, 25, 128] fp32 contiguous."""
     _chk(x); _chk(src)

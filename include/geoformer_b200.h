@@ -132,6 +132,29 @@ int gf_linattn_window_f16(const void* Q, int ldq, const void* K, int ldk, const 
                           int64_t n_windows, int tokens, int heads, int dim, gf_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * LoFTR full attention (`attention: 'full'`, loftr_module/linear_attention.py:54-85):
+ *   out[n,l,h,:] = softmax_s(Q[n,l,h,:] . K[n,s,h,:] / sqrt(dim)) V[n,s,h,:]
+ * on the plain projections (no elu+1 map).  Row strides ldq/ldk/ldv in elements; the message is fp32 [rows, heads*dim].
+ */
+/* coarse level, fp32 FFMA (accurate mode): q rows [n*l], k / v rows [n*s]; dim 32 */
+int gf_full_attention(const float* q, int ldq, const float* k, int ldk, const float* v, int ldv, float* out, int n, int l,
+                      int s, int heads, int dim, gf_stream_t stream);
+/* coarse level, tensor cores (fp16 operands, fp32 accumulate): gf_dense_kv_h16 lays the fp16 K / V rows [n*s]
+ * (8 heads of dim 32, 16-byte rows) out as kg[heads][n][s_pad][dim] and vt[heads][n][dim][s_pad] (zero for keys >= s,
+ * s_pad % 64 == 0) and sets key_cnt[n] = s; gf_full_attention_tc (dim 32) then runs the flash kernel of
+ * gf_geo_self_attention_tc over all s keys, reading the fp16 query rows in place through ldq. */
+int gf_dense_kv_h16(const void* k, int ldk, const void* v, int ldv, int n, int s, int heads, int dim, int s_pad, void* kg,
+                    void* vt, int* key_cnt, gf_stream_t stream);
+int gf_full_attention_tc(const void* q16, int ldq, const void* kg, const void* vt, const int* key_cnt, float* out, int n,
+                         int l, int s, int heads, int dim, int s_pad, gf_stream_t stream);
+/* fine level: windows of `tokens` (<= 32) rows attend to the paired window of the same index, heads x 16; one warp per
+ * (window, head).  Q / K / V fp32 or (_f16) fp16; the message is fp32 either way. */
+int gf_full_attention_window(const float* q, int ldq, const float* k, int ldk, const float* v, int ldv, float* out,
+                             int64_t n_windows, int tokens, int heads, int dim, gf_stream_t stream);
+int gf_full_attention_window_f16(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, float* out,
+                                 int64_t n_windows, int tokens, int heads, int dim, gf_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Coarse matching (utils/coarse_matching.py:110-125 and 161-212).
  * Split-fp16 operands: x*scale = hi + lo (fp16 each); role 0 (left operand) packs [hi | hi | lo],
  * role 1 (right operand) packs [hi | lo | hi] so that one K=3C fp16 tensor-core GEMM evaluates
